@@ -191,7 +191,7 @@ def dp_verify_batch(eng, rows, n_paths=48):
     return {"totals_equal_to_reference": ok_tot, "of": len(rows), "paths_equal_to_pinned_oracle": ok_path, "paths_checked": min(n_paths, len(rows))}
 
 
-def bench_dp(eng, torch, dist, world, rank, steps, warmup, l2_flush, stream, want_cpu):
+def bench_dp(eng, torch, dist, world, rank, steps, warmup, l2_flush, stream, want_cpu, dump=None):
     import ctypes as C
     from famsa_b200.binding import DpJob, DpProfile
     rows, jobs = dp_workload(rank)
@@ -234,6 +234,13 @@ def bench_dp(eng, torch, dist, world, rank, steps, warmup, l2_flush, stream, wan
         ev[s][1].record()
     barrier()
     launches = eng.kernel_launches() - l0
+    if dump is not None:                         # untimed: what the last timed step returned (DpResult records + paths)
+        res = d_res.cpu().numpy()
+        rec = res.view(np.int64).reshape(-1, 8)[:n]
+        poff, plen = res.view(np.uint64).reshape(-1, 8)[:n, 4], res.view(np.uint32).reshape(-1, 16)[:n, 12]
+        path = d_path.cpu().numpy()
+        dump["dp_total"] = rec[:, 0].astype(np.float64)
+        dump["dp_path"] = np.concatenate([path[int(o):int(o) + int(ln)] for o, ln in zip(poff, plen)]).astype(np.float32)
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -333,7 +340,7 @@ C3_N, C3_SEED = 100000, 2
 C5_N, C5_LEN, C5_SEEDS, C5_SEED = 3000000, 250, 100, 3
 
 
-def bench_c3(eng, torch, dist, world, rank, stream, l2_flush):
+def bench_c3(eng, torch, dist, world, rank, stream, l2_flush, steps):
     """BASELINE config 3 (strong scaling): the LCS triangle of 100 000 x 400 aa (4 999 950 000 pairs) sharded over the
     ranks, the exchange overlapped piece by piece; every rank ends with the full 10 GB packed triangle."""
     from famsa_b200 import seqio
@@ -349,7 +356,6 @@ def bench_c3(eng, torch, dist, world, rank, stream, l2_flush):
 
     step()
     dist.barrier(); torch.cuda.synchronize()
-    steps = 2
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for s in range(steps):
         l2_flush.fill_(s)
@@ -416,7 +422,7 @@ def c5_family(torch, n, L, seed):
     return codes.cpu().numpy().reshape(-1), offsets.cpu().numpy().astype(np.uint64), lens.cpu().numpy().astype(np.uint32)
 
 
-def bench_c5(eng, torch, dist, world, rank, stream, steps):
+def bench_c5(eng, torch, dist, world, rank, stream, steps, dump=None):
     """BASELINE config 5, the LCS side of -medoidtree: the assignment step of FastTree<>::makeEvaluation (FastTree.cpp:
     309-324) for 100 seeds x 3 000 000 sequences x 250 aa, the sequences sharded over the ranks, one NCCL MIN all-reduce of
     the packed (distance, seed) pairs."""
@@ -447,6 +453,9 @@ def bench_c5(eng, torch, dist, world, rank, stream, steps):
     out = None
     if rank == 0:
         a, d = unpack_assignment(packed.cpu().numpy())
+        if dump is not None:
+            dump["c5_assignment"] = a.astype(np.float32)
+            dump["c5_min_dist"] = d
         same = None
         if world > 1:                                # untimed: the unsharded call on this rank gives the same answer
             a1, d1 = eng.assign(seeds, 0)
@@ -497,7 +506,7 @@ def tree_workloads():
     return out
 
 
-def bench_dp_tree(eng, torch, dist, world, rank, steps, want_cpu):
+def bench_dp_tree(eng, torch, dist, world, rank, steps, want_cpu, dump=None):
     """Whole progressive alignments through famsa_prof_align_tree (one call per tree: every merge of the guide tree,
     profiles resident in HBM, per-merge records + paths back on the host), timed by the host clock around the call
     plus the path fetch.  Next to it the reference's own ComputeAlignment loop (CProfileQueue + worker threads) on all
@@ -528,6 +537,11 @@ def bench_dp_tree(eng, torch, dist, world, rank, steps, want_cpu):
             devs.append(st["device_ms"])
             eng.prof_drop([root])
         launches = eng.kernel_launches() - l0
+        if dump is not None:                      # what the last timed call returned: per-merge totals and paths
+            recs = raw["res"][:raw["n"]]
+            key = f"dp_tree{len(legs)}"
+            dump[key + "_total"] = np.array([r.total_score for r in recs], dtype=np.float64)
+            dump[key + "_path"] = np.concatenate([raw["path"][r.path_offset:r.path_offset + r.path_len] for r in recs]).astype(np.float32)
         wall = sorted(walls)[len(walls) // 2]
         t = torch.tensor([wall], dtype=torch.float64, device="cuda")
         if world > 1:
@@ -611,6 +625,31 @@ def run_reference(args):
     emit(line)
 
 
+DUMP_SAMPLE, DUMP_SEED, DUMP_LIMIT = 1 << 20, 12345, 64 << 20
+
+
+def dump_triangle(torch, tri_dev, total_pairs, dump):
+    """The packed uint16 LCS triangle of the last timed step: a fixed, seeded sample of DUMP_SAMPLE pairs (sorted
+    packed indices) and the sum over every pair."""
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total_pairs, size=min(DUMP_SAMPLE, total_pairs), replace=False))
+    t = tri_dev.view(torch.int16)[:total_pairs].to(torch.int32) & 0xFFFF
+    dump["lcs_triangle_index"] = idx.astype(np.float64)
+    dump["lcs_triangle_sample"] = t[torch.from_numpy(idx).cuda()].cpu().numpy().astype(np.float32)
+    dump["lcs_triangle_sum"] = np.array([t.to(torch.int64).sum().item()], dtype=np.float64)
+
+
+def write_dump(out_dir: str, dump: dict) -> dict:
+    """Writes every array as out_dir/<name>.npy; returns {name: shape} for the JSON line."""
+    total = sum(a.nbytes for a in dump.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dump.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "bytes": int(total), "arrays": {k: list(a.shape) for k, a in dump.items()}}
+
+
 _REAL_STDOUT = None
 
 
@@ -632,7 +671,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed legs computed in their last step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -651,6 +694,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 
     (codes, offsets, lens), n = workload(world)
+    dump = {} if args.dump_outputs and rank == 0 else None
     bounds = row_shards(n, world)
     rb, re = bounds[rank], bounds[rank + 1]
     my_pairs = tri(re) - tri(rb)
@@ -699,6 +743,8 @@ def main():
     barrier()
     wall1 = time.time()
     launches = eng.kernel_launches() - launches0
+    if dump is not None:
+        dump_triangle(torch, d_block if world == 1 else d_full, total_pairs, dump)
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -816,14 +862,14 @@ def main():
                 pairs = tri(n) - tri(n - n_s)
                 line["cpu_baseline"] = {"value": pairs / sec, "unit": UNIT, "cores": 1, "kind": "port",
                                         "sample": f"last {n_s} rows ({pairs} pairs)"}
-    dp = bench_dp(eng, torch, dist, world, rank, max(2, args.steps // 2), args.warmup, l2_flush, stream,
-                  want_cpu=(world == 1 and not args.no_cpu_baseline))
-    dp_tree = bench_dp_tree(eng, torch, dist, world, rank, max(3, args.steps), want_cpu=(world == 1 and not args.no_cpu_baseline))
+    dp = bench_dp(eng, torch, dist, world, rank, args.steps, args.warmup, l2_flush, stream,
+                  want_cpu=(world == 1 and not args.no_cpu_baseline), dump=dump)
+    dp_tree = bench_dp_tree(eng, torch, dist, world, rank, args.steps, want_cpu=(world == 1 and not args.no_cpu_baseline), dump=dump)
     if pt:
         d_full = None
         pt.close(torch)
-    c3 = bench_c3(eng, torch, dist, world, rank, stream, l2_flush) if world > 1 else None
-    c5 = bench_c5(eng, torch, dist, world, rank, stream, max(2, args.steps // 2))
+    c3 = bench_c3(eng, torch, dist, world, rank, stream, l2_flush, args.steps) if world > 1 else None
+    c5 = bench_c5(eng, torch, dist, world, rank, stream, args.steps, dump=dump)
     if rank == 0:
         line["dp"] = dp
         line["dp_tree"] = dp_tree
@@ -859,6 +905,8 @@ def main():
                                             "note": "UPGMA<indel075_div_lcs>::run of the bench set through famsa_lcs_upgma (no n^2 D2H)"}
             except Exception as e:
                 line["guide_tree_upgma"] = {"error": str(e)}
+        if dump is not None:
+            line["dump_outputs"] = write_dump(args.dump_outputs, dump)
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -11,7 +11,6 @@ from famsa_b200 import seqio
 from oracle import pyoracle
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 
 
 def assert_same(got, want, dirs=True):
@@ -32,7 +31,6 @@ def test_pp_golden(engine):
     assert_same(got, pyoracle.dp_align(*job, z["gaps"]))
 
 
-@needs_ref
 def test_all_merges_of_golden_upgma_tree(engine):
     """241 merges behind upgma.no_refine.fasta in ONE batch: every variant, oracle + reference + fixture."""
     z = np.load(os.path.join(GOLDEN, "adeno_upgma_merges.npz"))
@@ -47,7 +45,6 @@ def test_all_merges_of_golden_upgma_tree(engine):
         assert_same(r, pyoracle.dp_align(*rec["job"], g))
 
 
-@needs_ref
 @pytest.mark.parametrize("want_dirs", [False, True])
 def test_sub_batching(engine, monkeypatch, want_dirs):
     """Large batches are cut into sub-batches that bound the device scratch; force tiny ones."""
@@ -63,7 +60,6 @@ def test_sub_batching(engine, monkeypatch, want_dirs):
             assert np.array_equal(r["dirs"], pyoracle.dp_align(*rec["job"], g)["dirs"])
 
 
-@needs_ref
 def test_hemopexin_all_merges(engine):
     """BASELINE config 4: all 4187 guide-tree merges of test/hemopexin (medoid-sl tree) on one B200, level by
     level the way a host scheduler would submit them; totals and path CRCs pinned by the fixture, which was
@@ -85,7 +81,6 @@ def test_hemopexin_all_merges(engine):
     check_against_reference(engine.dp_align_batch([recs[k]["job"] for k in range(4000, 4187)], g), recs[4000:])
 
 
-@needs_ref
 @pytest.mark.parametrize("fixture", ["adeno_upgma_merges.npz", "hemopexin_medoid_sl.npz"])
 def test_gpu_driven_progressive_alignment(engine, fixture):
     """Drop-in proof for HP-2: the GPU's direction matrices and corner scores feed the reference's UNMODIFIED
@@ -104,7 +99,6 @@ def test_gpu_driven_progressive_alignment(engine, fixture):
     assert rows == recs[-1]["rows"]
 
 
-@needs_ref
 @pytest.mark.parametrize("seed,n,length,gaps", [(11, 70, 60, None), (12, 24, 500, None), (13, 40, 33, (-9000, -700, -300, -100)),
                                                 (14, 12, 1300, None), (15, 30, 31, (-20000, -2000, -2500, -900))])
 def test_random_families(engine, seed, n, length, gaps):
@@ -121,7 +115,6 @@ def test_random_families(engine, seed, n, length, gaps):
         assert_same(r, pyoracle.dp_align(*rec["job"], g))
 
 
-@needs_ref
 def test_cluster_path(engine, monkeypatch):
     """Very wide merges run on a thread-block cluster (8 blocks x 8 warps); force that path on ordinary sizes."""
     rng = np.random.default_rng(21)

@@ -10,6 +10,8 @@ from famsa_b200 import seqio
 from famsa_b200.binding import Engine
 from oracle import pyoracle
 
+import refgold
+
 pytestmark = pytest.mark.gpu
 
 
@@ -152,21 +154,25 @@ def test_full_size_properties(engine):
     assert int(tri.astype(np.uint64).sum()) == int(engine.triangle(dtype=np.uint16).astype(np.uint64).sum())
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 def test_full_c2_triangle_equals_reference(engine):
     """BASELINE config 2 in full: all 49 995 000 LCS lengths of the 10k x 400 aa set against the unmodified reference
-    (CLCSBP AVX2 through calculateDistanceVector, oracle/_ref) -- every pair, not a sample."""
+    (CLCSBP AVX2 through calculateDistanceVector, oracle/_ref; without it, the CRC32 of the reference's triangle)
+    -- every pair, not a sample."""
     codes, offsets, lens = seqio.synth_family(10000, 400, seed=1)
     n = len(lens)
-    letters = [seqio.decode(codes[int(o):int(o) + int(l)]) for o, l in zip(offsets, lens)]
-    rs = pyoracle.RefSeqSet(letters)
-    _, pairs, want = rs.triangle_mt(0, n, max(1, len(os.sched_getaffinity(0))), 2, want_lcs=True)
-    rs.close()
-    assert pairs == n * (n - 1) // 2
+
+    def reference():
+        letters = [seqio.decode(codes[int(o):int(o) + int(l)]) for o, l in zip(offsets, lens)]
+        rs = pyoracle.RefSeqSet(letters)
+        _, pairs, want = rs.triangle_mt(0, n, max(1, len(os.sched_getaffinity(0))), 2, want_lcs=True)
+        rs.close()
+        assert pairs == n * (n - 1) // 2
+        return want.astype(np.uint16)
+    want_crc = refgold.answer_crc("c2_triangle", reference)
     engine.upload(codes, offsets, lens)
     got = engine.triangle(dtype=np.uint16)
-    assert got.size == want.size
-    assert np.array_equal(got, want.astype(np.uint16)), "the C2 triangle differs from the reference's"
+    assert got.size == n * (n - 1) // 2
+    assert refgold.crc(got) == want_crc, "the C2 triangle differs from the reference's"
 
 
 def _assign_reference(codes, offsets, lens, seeds, kind, lcs_rows):
@@ -197,14 +203,16 @@ def test_medoid_assignment(engine, adeno, kind):
     got_a, got_d = engine.assign(seeds, kind)
     assert np.array_equal(got_a, want_a)
     assert np.array_equal(got_d.view(np.uint32), want_d.view(np.uint32))          # same float bits
-    if pyoracle.have_ref():
+    s = int(seeds[3])
+
+    def reference():
         rs = pyoracle.RefSeqSet(adeno["seqs"])
         lib = pyoracle.ref()
-        s = int(seeds[3])
         row = rs.row_prefix(s, len(lens), 2)
-        d = np.array([lib.ref_transform_f32(kind, int(row[j]), int(lens[s]), int(lens[j])) for j in range(len(lens))], dtype=np.float32)
-        assert np.all(got_d <= d)
-        assert np.array_equal(got_d[got_a == 3], d[got_a == 3])
+        return np.array([lib.ref_transform_f32(kind, int(row[j]), int(lens[s]), int(lens[j])) for j in range(len(lens))], dtype=np.float32)
+    d = refgold.answer(f"adeno/assign_row/{kind}/{s}", reference)
+    assert np.all(got_d <= d)
+    assert np.array_equal(got_d[got_a == 3], d[got_a == 3])
 
 
 def test_medoid_assignment_large(engine):
@@ -227,7 +235,6 @@ def test_medoid_assignment_large(engine):
     assert np.isfinite(cost)
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 def test_medoid_assignment_sharded(engine):
     """famsa_lcs_assign_shard: three shards of one context, combined with an element-wise MIN (what the NCCL all-reduce
     does across GPUs), equal the unsharded famsa_lcs_assign bit for bit -- ragged lengths, unsorted input, a repeated seed."""
@@ -263,12 +270,19 @@ def test_gpu_driven_upgma_tree(engine, modified):
     tri[i * (i - 1) // 2 + j] = [engine.transform(0, int(l), int(lens[a]), int(lens[b]), double=False)
                                  for l, a, b in zip(lcs[i * (i - 1) // 2 + j], i, j)]
     letters = [seqio.decode(codes[int(o):int(o) + int(ln)]) for o, ln in zip(offsets, lens)]
-    want = pyoracle.RefSeqSet(letters).upgma_tree(modified)
-    got = pyoracle.upgma_tree_from_distances(tri, n, modified)
-    assert np.array_equal(got, want)
+    if refgold.live():
+        want = pyoracle.RefSeqSet(letters).upgma_tree(modified)
+        got = pyoracle.upgma_tree_from_distances(tri, n, modified)
+        assert np.array_equal(got, want)
+
+    def reference_distances():                   # the reference's own LCS + Transform<float>: its UPGMA's input
+        _, _, ref_lcs = pyoracle.RefSeqSet(letters).triangle_mt(0, n, 4, 2, want_lcs=True)
+        f = pyoracle.ref().ref_transform_f32
+        return np.array([f(0, int(ref_lcs[i * (i - 1) // 2 + j]), int(lens[i]), int(lens[j])) for i, j in zip(*np.tril_indices(n, -1))],
+                        dtype=np.float32)
+    assert refgold.crc(tri) == refgold.answer_crc("upgma_driven/distances/" + refgold.input_key(letters), reference_distances)
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("modified", [False, True])
 @pytest.mark.parametrize("case", ["family400", "ragged", "big"])
 def test_device_upgma_tree(engine, modified, case):
@@ -287,7 +301,8 @@ def test_device_upgma_tree(engine, modified, case):
     engine.upload(codes, offsets, lens)
     got = engine.upgma(0, modified)
     letters = [seqio.decode(codes[int(o):int(o) + int(ln)]) for o, ln in zip(offsets, lens)]
-    want = pyoracle.RefSeqSet(letters).upgma_tree(modified, n_threads=8)[n:]
+    want = refgold.answer(f"upgma_tree/{case}/{int(modified)}/" + refgold.input_key(letters),
+                          lambda: pyoracle.RefSeqSet(letters).upgma_tree(modified, n_threads=8)[n:])
     assert got.shape == want.shape and np.array_equal(got, want)
 
 
@@ -367,11 +382,11 @@ def test_concurrent_callers_share_one_context(engine, adeno):
 from treeutil import prim_restated as _prim_restated  # noqa: E402
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("case", ["family", "adeno", "quirky", "tiny"])
 def test_gpu_prim_tree(engine, adeno, case):
     """Drop-in proof for the DEFAULT guide tree (-gt sl): famsa_lcs_prim's MST edges, passed to the reference's own
-    unmodified mst_to_dendogram, give exactly the tree MSTPrim<indel075_div_lcs> builds on the CPU."""
+    unmodified mst_to_dendogram, give exactly the tree MSTPrim<indel075_div_lcs> builds on the CPU.  Without oracle/_ref the
+    edges must be the ones that were checked to give that tree when the stored answers were recorded."""
     if case == "family":
         codes, offsets, lens = seqio.synth_family(700, 130, seed=41)
     elif case == "adeno":
@@ -389,10 +404,17 @@ def test_gpu_prim_tree(engine, adeno, case):
     engine.upload(codes, offsets, lens)
     ef, et, ed, order = engine.prim(0)
     letters = [seqio.decode(codes[int(o):int(o) + int(ln)]) for o, ln in zip(offsets, lens)]
-    want = pyoracle.RefSeqSet(letters).mst_prim_tree(3)
-    got = pyoracle.mst_to_dendogram(ef, et, ed, order)
-    assert np.array_equal(got, want)
+    if refgold.live():
+        want = pyoracle.RefSeqSet(letters).mst_prim_tree(3)
+        got = pyoracle.mst_to_dendogram(ef, et, ed, order)
+        assert np.array_equal(got, want)
+    assert refgold.crc(_edges(ef, et, ed, order)) == refgold.answer_crc(f"prim_tree/{case}/" + refgold.input_key(letters),
+                                                                        lambda: _edges(ef, et, ed, order))
     assert sorted(order.tolist()) == list(range(n))
+
+
+def _edges(ef, et, ed, order):
+    return np.concatenate([np.asarray(x, dtype=np.float64) for x in (ef, et, ed, order)])
 
 
 @pytest.mark.parametrize("sequential", [False, True])
@@ -425,12 +447,12 @@ def test_gpu_prim_golden_sl_tree(engine, monkeypatch, sequential):
     assert np.array_equal(ed, z["edge_dist"]) and np.array_equal(order, z["prim_order"])
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 def test_gpu_prim_lrr_golden_tree():
     """The reference's large default-guide-tree golden, test/LRR/sl.dnd (124 140 sequences; fixture lrr_sl.npz: the set in
     FAMSA's order and the CRC of the reference's MSTPrim tree, whose clades were checked against sl.dnd at generation).
     famsa_lcs_prim keeps the 7.7 G-pair triangle in HBM (15 GB as u16 + 62 GB of float64 distances for the Boruvka
-    rounds); its edges, through the reference's own mst_to_dendogram, must give that tree."""
+    rounds); its edges, through the reference's own mst_to_dendogram, must give that tree (without oracle/_ref: must be
+    the edges that were checked to give it when the stored answers were recorded)."""
     path = os.path.join(GOLDEN, "lrr_sl.npz")
     if not os.path.exists(path):
         pytest.skip("lrr_sl.npz not generated")
@@ -445,8 +467,10 @@ def test_gpu_prim_lrr_golden_tree():
         ef, et, ed, order = eng.prim(0)
     finally:
         eng.close()
-    tree = pyoracle.mst_to_dendogram(ef, et, ed, order)
-    assert zlib.crc32(np.ascontiguousarray(tree[n:], dtype=np.int32).tobytes()) == int(z["tree_crc"][0])
+    if refgold.live():
+        tree = pyoracle.mst_to_dendogram(ef, et, ed, order)
+        assert zlib.crc32(np.ascontiguousarray(tree[n:], dtype=np.int32).tobytes()) == int(z["tree_crc"][0])
+    assert refgold.crc(_edges(ef, et, ed, order)) == refgold.answer_crc("prim_tree/lrr", lambda: _edges(ef, et, ed, order))
 
 
 def test_gpu_prim_lower_bound_pruning_case(engine):

@@ -10,7 +10,6 @@ from dp_cases import check_against_reference, random_tree, reference_merges
 from famsa_b200 import seqio
 from oracle import pyoracle
 
-needs_ref = pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 
 
 def test_oracle_pp_golden():
@@ -24,7 +23,6 @@ def test_oracle_pp_golden():
     assert np.all(d[0, 1:] == 0x15) and np.all(d[1:, 0] == 0x2A) and d[0, 0] == 0
 
 
-@needs_ref
 def test_oracle_all_merges_of_golden_upgma_tree():
     """All 241 merges (SeqSeq, SeqProf, ProfProf) behind test/adeno_fiber/upgma.no_refine.fasta."""
     z = np.load(os.path.join(GOLDEN, "adeno_upgma_merges.npz"))
@@ -39,7 +37,6 @@ def test_oracle_all_merges_of_golden_upgma_tree():
     assert sorted(set(r["variant"] for r in res)) == [0, 1, 2]
 
 
-@needs_ref
 @pytest.mark.parametrize("seed,n,length,gaps", [(1, 60, 90, None), (2, 40, 300, None), (3, 50, 40, (-9000, -700, -300, -100)),
                                                 (4, 30, 150, (-20000, -2000, -2500, -900))])
 def test_oracle_random_families(seed, n, length, gaps):
@@ -58,7 +55,6 @@ def test_oracle_hemopexin_fixture_selfcheck():
     assert len(z["seqs"]) == 4188 and len(z["merges"]) == 4187 and len(z["totals"]) == 4187
 
 
-@needs_ref
 def test_oracle_hemopexin_first_levels():
     """Config 4 subset on CPU (the whole tree runs in the GPU test): first 400 merges of medoid-sl.dnd."""
     z = np.load(os.path.join(GOLDEN, "hemopexin_medoid_sl.npz"))
@@ -85,7 +81,6 @@ def test_oracle_hemopexin_first_levels():
     _check_construct(res, recs, g)               # and the merged tables ConstructProfile builds from those paths
 
 
-@needs_ref
 def test_oracle_driven_alignment_equals_reference():
     """The oracle's direction matrices drive the reference's own ConstructProfile through the whole upgma tree of
     adeno_fiber: the final alignment must be the reference's, row for row."""
@@ -119,7 +114,6 @@ def _check_construct(res, recs, g):
             assert all(not mask[a - 1] and not mask[a + ln] for a, ln in runs), "runs must be maximal"
 
 
-@needs_ref
 def test_oracle_construct_golden_upgma_tree():
     """Merged profile tables after each of the 241 merges behind upgma.no_refine.fasta (ConstructProfile,
     profile.cpp:784-1002) -- the widened row SURVEY 8f-2."""
@@ -131,7 +125,6 @@ def test_oracle_construct_golden_upgma_tree():
     _check_construct(res, recs, g)
 
 
-@needs_ref
 @pytest.mark.parametrize("seed,n,length,gaps", [(11, 50, 80, None), (12, 40, 200, (-9000, -700, -300, -100))])
 def test_oracle_construct_random_families(seed, n, length, gaps):
     rng = np.random.default_rng(seed)

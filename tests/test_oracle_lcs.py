@@ -7,6 +7,8 @@ from conftest import QUIRK_LCS, QUIRK_SEQS, random_set
 from famsa_b200 import seqio
 from oracle import pyoracle
 
+import refgold
+
 
 def test_oracle_matches_golden_pid_sq(adeno):
     """Every one of the 242 x 242 exact LCS lengths pinned by test/adeno_fiber/pid_sq.csv."""
@@ -45,10 +47,6 @@ def test_oracle_distance_golden(adeno):
             assert abs(d - adeno["dist"][i, j]) < 1e-6 * max(1.0, abs(d)) + 6e-7
 
 
-needs_ref = pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
-
-
-@needs_ref
 @pytest.mark.parametrize("isa", [0, 2])
 def test_oracle_vs_reference_random(isa):
     rng = np.random.default_rng(5)
@@ -57,38 +55,51 @@ def test_oracle_vs_reference_random(isa):
     code_list.append(np.zeros(200, np.int8))                          # quirky: 'A' * 200
     code_list.append(np.concatenate([np.zeros(64, np.int8), np.ones(70, np.int8)]))
     letters = [seqio.decode(c) for c in code_list]
-    rs = pyoracle.RefSeqSet(letters)
-    assert all(np.array_equal(a, b) for a, b in zip(rs.codes(), code_list))
+    rs = pyoracle.RefSeqSet(letters) if refgold.live() else None
+    key = f"lcs_random/{isa}/" + refgold.input_key(letters)
     codes, offsets, lens = seqio.pack(code_list)
+    assert refgold.crc(codes) == refgold.answer_crc(key + "/codes", lambda: np.concatenate(rs.codes()))
     n = len(code_list)
+    want = refgold.answer(key + "/rows", lambda: np.stack([rs.row_prefix(r, n, isa) for r in range(n)]).astype(np.uint16))
     for r in range(n):
-        want = rs.row_prefix(r, n, isa)
         got = pyoracle.lcs_rows(codes, offsets, lens, [r])[0]
-        assert np.array_equal(got, want), f"row {r}"
+        assert np.array_equal(got, want[r]), f"row {r}"
     ids = rng.permutation(n)[:37]
-    assert np.array_equal(rs.row_ids(3, ids, isa), pyoracle.lcs_rows(codes, offsets, lens, [3], ids)[0])
+    want = refgold.answer(key + "/ids", lambda: rs.row_ids(3, ids, isa).astype(np.uint16))
+    assert np.array_equal(want, pyoracle.lcs_rows(codes, offsets, lens, [3], ids)[0])
 
 
-@needs_ref
 def test_reference_reproduces_golden(adeno):
-    """The compiled reference (AVX2 path) reproduces its own pid_sq.csv through the harness."""
-    rs = pyoracle.RefSeqSet(adeno["seqs"])
+    """The compiled reference (AVX2 path) reproduces its own pid_sq.csv through the harness (without oracle/_ref: the
+    reference's stored answers do)."""
+    rs = pyoracle.RefSeqSet(adeno["seqs"]) if refgold.live() else None
     n = len(adeno["lens"])
-    for r in range(0, n, 9):
-        assert np.array_equal(rs.row_prefix(r, n, 2), adeno["lcs"][r])
-    sec, pairs, tri = rs.triangle_mt(0, n, 4, 2, want_lcs=True)
+    rows = refgold.answer("adeno/rows_every_9th", lambda: np.stack([rs.row_prefix(r, n, 2) for r in range(0, n, 9)]).astype(np.uint16))
+    assert np.array_equal(rows, adeno["lcs"][0:n:9])
     i, j = np.tril_indices(n, -1)
-    assert pairs == n * (n - 1) // 2
-    assert np.array_equal(tri[i * (i - 1) // 2 + j], adeno["lcs"][i, j])
+    want = adeno["lcs"][i, j].astype(np.uint32)
+
+    def triangle():
+        sec, pairs, tri = rs.triangle_mt(0, n, 4, 2, want_lcs=True)
+        assert pairs == n * (n - 1) // 2
+        return tri
+    assert refgold.crc(want) == refgold.answer_crc("adeno/triangle", triangle)
 
 
-@needs_ref
 def test_transform_vs_reference():
-    lib = pyoracle.ref()
     rng = np.random.default_rng(1)
+    args = []
     for _ in range(300):
         l1, l2 = (int(x) for x in rng.integers(1, 600, size=2))
         lcs = int(rng.integers(0, min(l1, l2) + 1))
-        for kind in (0, 1, 2):
-            assert pyoracle.transform(kind, lcs, l1, l2, True) == lib.ref_transform_f64(kind, lcs, l1, l2)
-            assert pyoracle.transform(kind, lcs, l1, l2, False) == lib.ref_transform_f32(kind, lcs, l1, l2)
+        args += [(kind, lcs, l1, l2) for kind in (0, 1, 2)]
+
+    def reference(f64):
+        lib = pyoracle.ref()
+        f = lib.ref_transform_f64 if f64 else lib.ref_transform_f32
+        return np.array([f(*a) for a in args], dtype=np.float64 if f64 else np.float32)
+    want64 = refgold.answer("transform/f64", lambda: reference(True))
+    want32 = refgold.answer("transform/f32", lambda: reference(False))
+    for a, w64, w32 in zip(args, want64, want32):
+        assert pyoracle.transform(*a, True) == w64
+        assert pyoracle.transform(*a, False) == w32

@@ -8,13 +8,13 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN
-from dp_cases import check_against_reference, random_tree, reference_merges, resident_progressive_alignment
+from dp_cases import (check_against_reference, random_tree, reference_merges, reference_score_matrix,
+                      resident_progressive_alignment)
 from famsa_b200 import seqio
 from famsa_b200.binding import PROF_LEAF, Engine, FamsaError
 from oracle import pyoracle
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 
 
 @pytest.fixture(scope="module")
@@ -25,10 +25,7 @@ def engine():
 
 
 def _score_matrix(n):
-    dp = pyoracle.RefDp(n)
-    sm = dp.score_matrix()
-    dp.close()
-    return sm
+    return reference_score_matrix(n)
 
 
 def _run_and_check(engine, seqs, merges, g, recs, sm):
@@ -53,7 +50,6 @@ def _run_and_check(engine, seqs, merges, g, recs, sm):
     return results
 
 
-@needs_ref
 def test_resident_golden_upgma_tree(engine):
     """All 241 merges behind test/adeno_fiber/upgma.no_refine.fasta with profiles resident in HBM."""
     z = np.load(os.path.join(GOLDEN, "adeno_upgma_merges.npz"))
@@ -65,7 +61,6 @@ def test_resident_golden_upgma_tree(engine):
     assert np.array_equal(np.concatenate([r["path"] for r in res]), z["path"])
 
 
-@needs_ref
 @pytest.mark.parametrize("seed,n,length,gaps,cat", [(31, 60, 70, None, 0.3), (32, 24, 400, None, 0.6),
                                                     (33, 40, 33, (-9000, -700, -300, -100), 0.2),
                                                     (34, 10, 1300, None, 0.5)])
@@ -79,7 +74,6 @@ def test_resident_random_families(engine, seed, n, length, gaps, cat):
     _run_and_check(engine, seqs, merges, g, recs, _score_matrix(n))
 
 
-@needs_ref
 def test_resident_hemopexin(engine):
     """4188 sequences / 94 levels (golden medoid-sl tree): totals and path checksums of every merge, and the final
     alignment assembled from the paths, equal the fixture the reference generated."""
@@ -97,7 +91,6 @@ def test_resident_hemopexin(engine):
     assert engine.prof_stats() == (0, 0)
 
 
-@needs_ref
 def test_prof_put_and_mixed_children(engine):
     """Host-built tables uploaded with famsa_prof_put merge exactly like the reference's; leaf + resident mixes."""
     rng = np.random.default_rng(5)
@@ -152,7 +145,6 @@ def test_prof_errors(engine):
     assert engine.prof_stats() == (0, 0)
 
 
-@needs_ref
 @pytest.mark.parametrize("env", [{"FAMSA_PROF_FUSED": "0", "FAMSA_DP_MAX_CELLS": "60000"},
                                  {"FAMSA_PROF_FUSED": "0", "FAMSA_DP_LATENCY_MODE": "0", "FAMSA_DP_CLUSTER_MIN": "40", "FAMSA_DP_TEAM_MIN": "32"},
                                  {"FAMSA_PROF_FUSED": "0", "FAMSA_DP_LATENCY_MODE": "0", "FAMSA_DP_TEAM_MIN": "100000"},

@@ -167,21 +167,20 @@ def _tree_worker(rank, world, port, n, out_dir):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(not pyoracle.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("world", [2, 3])
 def test_subtree_sharded_resident_alignment(tmp_path, world):
     """HP-2 on several ranks with resident profiles: whole subtrees per rank (no communication), subtree roots handed
     to rank 0, top merges there.  Every merge runs exactly once and the assembled alignment is the reference's."""
     import sys
     sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    from dp_cases import assemble_rows, random_tree, reference_merges
+    from dp_cases import assemble_rows, random_tree, reference_merges, reference_score_matrix
     n = 26
     rng = np.random.default_rng(8)
     codes, off, lens = seqio.synth_family(n, 45, 8, sort_desc=False)
     seqs = [seqio.decode(codes[int(o):int(o) + int(l)]) for o, l in zip(off, lens)]
     merges = random_tree(n, rng, 0.3)
     g, recs = reference_merges(seqs, merges, threads=(1,))
-    dp = pyoracle.RefDp(n); sm = dp.score_matrix(); dp.close()
+    sm = reference_score_matrix(n)
     np.savez(tmp_path / "case.npz", seqs=np.array(seqs), merges=np.array(merges), sm=sm, gaps=g)
     port = 29640 + world
     mp.spawn(_tree_worker, args=(world, port, n, str(tmp_path)), nprocs=world, join=True)
