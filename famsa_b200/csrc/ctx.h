@@ -26,6 +26,14 @@ const char* get_error();
         }                                                                                    \
     } while (0)
 
+#define FB_TRY(expr)                       \
+    do {                                   \
+        int rc__ = (expr);                 \
+        if (rc__ != FAMSA_OK) return rc__; \
+    } while (0)
+
+struct FusedParams;   // prof_dev.cuh
+
 // Simple owning device buffer that only grows.
 struct DevBuf {
     void* p = nullptr;
@@ -62,6 +70,7 @@ struct LcsState {
     float last_total_ms = 0.f, last_main_ms = 0.f;
     uint64_t last_pairs = 0;
     uint64_t last_tiles = 0;                 // tiles launched by the most recent triangle call
+    uint64_t tile_configured = 0;            // bit NL-1: k_lcs_tile<NL> has its shared-memory attribute on this device
     std::vector<uint32_t> h_order;           // famsa_lcs_upload_sorted: position in the library's order -> caller index
 };
 
@@ -71,6 +80,9 @@ struct DpState {
     size_t h_pinned_cap = 0;
     uint64_t last_cells = 0;
     float last_total_ms = 0.f, last_kernel_ms = 0.f;
+    // kernel attributes of the fill and fused kernels are set, and the cluster caps probed, on the first DP call
+    bool configured = false;
+    uint32_t cluster4_cap = 1, duo_cap = 1;   // largest cluster of k_dp_fill<4, true> / k_dp_fill_duo blocks
 };
 
 // Profiles kept resident in HBM between the levels of the guide tree (prof.cu).
@@ -229,16 +241,15 @@ int dp_run_host(famsa_ctx* ctx, const famsa_dp_job* jobs, uint32_t n, const int6
                 uint8_t* path_buf, uint8_t* dirs_buf);
 int dp_check_results(const famsa_dp_result* results, uint32_t n);
 // d_meta_out / d_blob_out non-NULL: the per-job DpMeta records stay valid until the caller cudaFreeAsync()s *d_blob_out
-// fused non-NULL (a FusedParams, prof_dev.cuh): every merge runs whole -- leaves, prep, fill, traceback, merged tables --
-// in one block of k_merge_fused; the caller then launches neither the leaf nor the construct kernel.
 int dp_run_device(famsa_ctx* ctx, const famsa_dp_job* jobs, const DpJobExt* ext, uint32_t n, const int64_t gaps[4],
                   famsa_dp_result* d_results, uint8_t* d_path, uint8_t* d_dirs, DpMeta** d_meta_out, void** d_blob_out,
-                  cudaStream_t st, const void* fused = nullptr);
+                  cudaStream_t st);
 int dp_fused_plan(const famsa_dp_job* jobs, const DpJobExt* ext, uint32_t n, bool align16, DpJobDev* out, DpFusedPlan* plan);
 int dp_fused_launch(famsa_ctx* ctx, const DpJobDev* jobs, uint32_t n, const int64_t gaps[4], famsa_dp_result* d_results, uint8_t* d_path,
                     DpMeta* d_meta, uint8_t* d_scratch, uint8_t* d_skew, famsa_dp_result* h_results, uint8_t* h_path,
-                    const void* fused_params, uint32_t grid, uint64_t cells, bool record_events, cudaStream_t st);
+                    const FusedParams& fused, uint32_t grid, uint64_t cells, bool record_events, cudaStream_t st);
 unsigned long long dp_scratch_bytes(uint32_t w1, uint32_t w2);
+bool dp_debug();   // FAMSA_DP_DEBUG (development aid, read once per process): launch decisions go to stderr
 // prof.cu
 int prof_set_scoring(famsa_ctx* ctx, const int64_t* sm);
 int prof_put(famsa_ctx* ctx, const famsa_dp_profile* profs, uint32_t n, uint32_t* ids);

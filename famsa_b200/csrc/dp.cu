@@ -27,7 +27,6 @@
 //              per step).  The same kernel then walks the direction matrix back and emits the path.
 //   k_dp_unskew only when the caller asks for CDPMatrix bytes: skewed directions -> row-major.
 #include <algorithm>
-#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -1332,118 +1331,143 @@ extern "C" int famsa_debug_fused_phases(double out_ns[8])
 // host side
 // ------------------------------------------------------------------------------------------------
 
-#define FB_TRY(expr)                      \
-    do {                                  \
-        int rc__ = (expr);                \
-        if (rc__ != FAMSA_OK) return rc__; \
-    } while (0)
+using FillKernel = void (*)(DpParams);
 
-template <int NW, bool CLUSTERED>
-static int configure_fill(famsa_ctx* ctx)
+// largest cluster size in {2, 4, 8, 16} that `kernel` can be launched with on this device (1: none)
+static uint32_t max_cluster(FillKernel kernel, int block, size_t smem)
 {
-    static std::atomic<bool> configured[64];
-    constexpr int warps = NW == 1 ? kDpWarps : NW;
-    if (!configured[ctx->device & 63].load(std::memory_order_acquire)) {
-        FB_CUDA(cudaFuncSetAttribute(k_dp_fill<NW, CLUSTERED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(warps * sizeof(WarpShared))));
-        if (CLUSTERED) FB_CUDA(cudaFuncSetAttribute(k_dp_fill<NW, CLUSTERED>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        configured[ctx->device & 63].store(true, std::memory_order_release);
-    }
-    return FAMSA_OK;
-}
-
-template <int NW>
-static int launch_cluster_fill(famsa_ctx* ctx, const DpParams& Q, uint32_t cl, cudaStream_t st)
-{
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(Q.n_jobs * cl);
-    cfg.blockDim = dim3(NW * 32);
-    cfg.dynamicSmemBytes = NW * sizeof(WarpShared);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    FB_CUDA(cudaLaunchKernelEx(&cfg, k_dp_fill<NW, true>, Q));
-    ctx->launches++;
-    return FAMSA_OK;
-}
-
-static int launch_duo_fill(famsa_ctx* ctx, const DpParams& Q, uint32_t cl, cudaStream_t st)
-{
-    static std::atomic<bool> configured[64];
-    if (!configured[ctx->device & 63].load(std::memory_order_acquire)) {
-        FB_CUDA(cudaFuncSetAttribute(k_dp_fill_duo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDuoSmem));
-        FB_CUDA(cudaFuncSetAttribute(k_dp_fill_duo, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        configured[ctx->device & 63].store(true, std::memory_order_release);
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(Q.n_jobs * cl);
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = kDuoSmem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    FB_CUDA(cudaLaunchKernelEx(&cfg, k_dp_fill_duo, Q));
-    ctx->launches++;
-    return FAMSA_OK;
-}
-
-// largest cluster size (<= 16) the duo kernel (one block per SM) can be launched with on this device
-static uint32_t max_cluster_duo(famsa_ctx* ctx)
-{
-    static std::atomic<int> cached[64];
-    int v = cached[ctx->device & 63].load(std::memory_order_acquire);
-    if (v) return (uint32_t)v;
-    cudaFuncSetAttribute(k_dp_fill_duo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDuoSmem);
-    cudaFuncSetAttribute(k_dp_fill_duo, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    v = 1;
-    for (int cl : {2, 4, 8, 16}) {
+    uint32_t v = 1;
+    for (uint32_t cl : {2u, 4u, 8u, 16u}) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(cl);
-        cfg.blockDim = dim3(256);
-        cfg.dynamicSmemBytes = kDuoSmem;
+        cfg.blockDim = dim3(block);
+        cfg.dynamicSmemBytes = smem;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeClusterDimension;
         attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
         int n = 0;
-        if (cudaOccupancyMaxActiveClusters(&n, k_dp_fill_duo, &cfg) == cudaSuccess && n > 0) v = cl;
-        else { cudaGetLastError(); break; }
+        if (cudaOccupancyMaxActiveClusters(&n, kernel, &cfg) != cudaSuccess || n == 0) { cudaGetLastError(); break; }
+        v = cl;
     }
-    cached[ctx->device & 63].store(v, std::memory_order_release);
-    return (uint32_t)v;
+    return v;
 }
 
-// largest cluster size (<= 16) the 4-warp fill kernel can be launched with on this device
-static uint32_t max_cluster4(famsa_ctx* ctx)
+// Kernel attributes of every fill shape and of k_merge_fused, and the cluster caps: once per context, on the first DP
+// call (an LCS-only caller never loads the DP kernels).
+static int configure_dp(famsa_ctx* ctx)
 {
-    static std::atomic<int> cached[64];
-    int v = cached[ctx->device & 63].load(std::memory_order_acquire);
-    if (v) return (uint32_t)v;
-    v = 8;
-    for (int cl : {16}) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(cl);
-        cfg.blockDim = dim3(4 * 32);
-        cfg.dynamicSmemBytes = 4 * sizeof(WarpShared);
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        int n = 0;
-        if (cudaOccupancyMaxActiveClusters(&n, k_dp_fill<4, true>, &cfg) == cudaSuccess && n > 0) v = cl;
-        else cudaGetLastError();
+    DpState& S = ctx->dp;
+    if (S.configured) return FAMSA_OK;
+    const auto smem = [](auto kernel, size_t bytes) {
+        return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    };
+    const auto any_cluster = [](auto kernel) {
+        return cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    };
+    FB_CUDA(smem(k_dp_fill<1, false>, kDpWarps * sizeof(WarpShared)));
+    FB_CUDA(smem(k_dp_fill<2, false>, 2 * sizeof(WarpShared)));
+    FB_CUDA(smem(k_dp_fill<4, false>, 4 * sizeof(WarpShared)));
+    FB_CUDA(smem(k_dp_fill<kDpTeamWarps, false>, kDpTeamWarps * sizeof(WarpShared)));
+    FB_CUDA(smem(k_dp_fill<4, true>, 4 * sizeof(WarpShared)));
+    FB_CUDA(any_cluster(k_dp_fill<4, true>));
+    FB_CUDA(smem(k_dp_fill<kDpTeamWarps, true>, kDpTeamWarps * sizeof(WarpShared)));
+    FB_CUDA(any_cluster(k_dp_fill<kDpTeamWarps, true>));
+    FB_CUDA(smem(k_dp_fill_duo, kDuoSmem));
+    FB_CUDA(any_cluster(k_dp_fill_duo));
+    FB_CUDA(smem(k_dp_fill_compact<2>, 2 * kCompactStride));
+    FB_CUDA(smem(k_dp_fill_compact<4>, 4 * kCompactStride));
+    FB_CUDA(smem(k_dp_fill_compact<6>, 6 * kCompactStride));
+    FB_CUDA(smem(k_merge_fused, kFusedWarps * sizeof(WarpShared)));
+    S.cluster4_cap = max_cluster(k_dp_fill<4, true>, 4 * 32, 4 * sizeof(WarpShared));
+    S.duo_cap = max_cluster(k_dp_fill_duo, 256, kDuoSmem);
+    S.configured = true;
+    return FAMSA_OK;
+}
+
+// Every fill launch: `grid` blocks, in clusters of `cl` blocks when cl > 1.
+static int launch_fill(famsa_ctx* ctx, FillKernel kernel, const DpParams& Q, uint32_t grid, uint32_t block,
+                       size_t smem, uint32_t cl, cudaStream_t st)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = cl > 1 ? 1 : 0;
+    FB_CUDA(cudaLaunchKernelEx(&cfg, kernel, Q));
+    ctx->launches++;
+    return FAMSA_OK;
+}
+
+// Development knobs of the fill launch policy.  Read on every dp_run_device call: tests change them between calls.
+struct DpKnobs {
+    unsigned long long max_cells = 1ull << 32;     // FAMSA_DP_MAX_CELLS: matrix cells per sub-batch
+    uint32_t team_min = kDpTeamMinWidth;           // FAMSA_DP_TEAM_MIN
+    int team_warps = 0;                            // FAMSA_DP_TEAM_WARPS (0: by the number of merges)
+    uint32_t cluster_min = kDpClusterMinWidth;     // FAMSA_DP_CLUSTER_MIN
+    uint32_t max_cluster = 0xffffffffu;            // FAMSA_DP_MAX_CLUSTER: limits the probed cap
+    int latency_mode = -1;                         // FAMSA_DP_LATENCY_MODE (-1: by the batch's demand)
+    bool duo = true;                               // FAMSA_DP_DUO=0: one warp per stripe instead of producer / consumer pairs
+    int compact = 1;                               // FAMSA_DP_COMPACT: 0 never, 1 from two merges per SM on, 2 always
+};
+
+static DpKnobs read_knobs()
+{
+    DpKnobs K;
+    if (const char* e = getenv("FAMSA_DP_MAX_CELLS")) K.max_cells = strtoull(e, nullptr, 10);
+    if (const char* e = getenv("FAMSA_DP_TEAM_MIN")) K.team_min = (uint32_t)atoi(e);
+    if (const char* e = getenv("FAMSA_DP_TEAM_WARPS")) K.team_warps = atoi(e);
+    if (const char* e = getenv("FAMSA_DP_CLUSTER_MIN")) K.cluster_min = (uint32_t)atoi(e);
+    if (const char* e = getenv("FAMSA_DP_MAX_CLUSTER")) K.max_cluster = (uint32_t)atoi(e);
+    if (const char* e = getenv("FAMSA_DP_LATENCY_MODE")) K.latency_mode = atoi(e) != 0;
+    if (const char* e = getenv("FAMSA_DP_DUO")) K.duo = atoi(e) != 0;
+    if (const char* e = getenv("FAMSA_DP_COMPACT")) K.compact = atoi(e);
+    return K;
+}
+
+bool dp_debug()
+{
+    static const bool debug = getenv("FAMSA_DP_DEBUG") != nullptr;
+    return debug;
+}
+
+// Job k as the kernels see it, without its buffer offsets.  jobs[k].p1/p2 hold DEVICE pointers; the widths are the
+// layout widths (upper bounds when ext->w*_src is set).
+static int make_job(const famsa_dp_job& j, const DpJobExt* ext, uint32_t k, DpJobDev& d)
+{
+    if (j.p1.width == 0 || j.p2.width == 0 || j.p1.card == 0 || j.p2.card == 0) {
+        set_error("dp job " + std::to_string(k) + ": empty profile");
+        return FAMSA_E_INVALID;
     }
-    cached[ctx->device & 63].store(v, std::memory_order_release);
-    return (uint32_t)v;
+    if (((unsigned long long)j.p1.width + 1) * (j.p2.width + 1) > 0xffffffffull) {
+        set_error("dp job " + std::to_string(k) + ": more than 2^32 matrix cells");
+        return FAMSA_E_INVALID;
+    }
+    d.s1 = reinterpret_cast<const long long*>(j.p1.scores); d.c1 = j.p1.counters;
+    d.s2 = reinterpret_cast<const long long*>(j.p2.scores); d.c2 = j.p2.counters;
+    d.w1 = j.p1.width; d.card1 = j.p1.card; d.w2 = j.p2.width; d.card2 = j.p2.card;
+    d.w1_src = ext ? ext->w1_src : nullptr; d.w2_src = ext ? ext->w2_src : nullptr; d.w_dst = ext ? ext->w_dst : nullptr;
+    return FAMSA_OK;
+}
+
+// what every launch of one batch shares
+static DpParams batch_params(const DpJobDev* jobs, DpMeta* meta, const int64_t gaps[4], uint8_t* sdirs, uint8_t* path,
+                             uint8_t* scratch, famsa_dp_result* results)
+{
+    DpParams P{};
+    P.jobs = jobs;
+    P.meta = meta;
+    P.go = gaps[0]; P.ge = gaps[1]; P.to = gaps[2]; P.te = gaps[3];
+    P.sdirs = sdirs;
+    P.path = path;
+    P.scratch = scratch;
+    P.results = results;
+    return P;
 }
 
 unsigned long long dp_scratch_bytes(uint32_t w1, uint32_t w2) { return Scratch(w1, w2).total; }
@@ -1454,13 +1478,8 @@ int dp_fused_plan(const famsa_dp_job* jobs, const DpJobExt* ext, uint32_t n, boo
 {
     unsigned long long path_off = 0, scratch_off = 0, t_off = 0, cells = 0;
     for (uint32_t k = 0; k < n; ++k) {
-        const famsa_dp_job& j = jobs[k];
-        if (j.p1.width == 0 || j.p2.width == 0 || j.p1.card == 0 || j.p2.card == 0) { set_error("dp job " + std::to_string(k) + ": empty profile"); return FAMSA_E_INVALID; }
         DpJobDev& d = out[k];
-        d.s1 = reinterpret_cast<const long long*>(j.p1.scores); d.c1 = j.p1.counters;
-        d.s2 = reinterpret_cast<const long long*>(j.p2.scores); d.c2 = j.p2.counters;
-        d.w1 = j.p1.width; d.card1 = j.p1.card; d.w2 = j.p2.width; d.card2 = j.p2.card;
-        d.w1_src = ext ? ext[k].w1_src : nullptr; d.w2_src = ext ? ext[k].w2_src : nullptr; d.w_dst = ext ? ext[k].w_dst : nullptr;
+        FB_TRY(make_job(jobs[k], ext ? ext + k : nullptr, k, d));
         d.path_off = path_off; d.dirs_off = 0;
         d.scratch_off = scratch_off; d.t_off = t_off;
         path_off += align16 ? align_up((unsigned long long)d.w1 + d.w2, 16) : (unsigned long long)d.w1 + d.w2;   // 16-byte slots: the traceback
@@ -1475,96 +1494,46 @@ int dp_fused_plan(const famsa_dp_job* jobs, const DpJobExt* ext, uint32_t n, boo
 
 int dp_fused_launch(famsa_ctx* ctx, const DpJobDev* jobs, uint32_t n, const int64_t gaps[4], famsa_dp_result* d_results, uint8_t* d_path,
                     DpMeta* d_meta, uint8_t* d_scratch, uint8_t* d_skew, famsa_dp_result* h_results, uint8_t* h_path,
-                    const void* fused_params, uint32_t grid, uint64_t cells, bool record_events, cudaStream_t st)
+                    const FusedParams& fused, uint32_t grid, uint64_t cells, bool record_events, cudaStream_t st)
 {
-    static std::atomic<bool> configured[64];
-    if (!configured[ctx->device & 63].load(std::memory_order_acquire)) {
-        FB_CUDA(cudaFuncSetAttribute(k_merge_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kFusedWarps * sizeof(WarpShared))));
-        configured[ctx->device & 63].store(true, std::memory_order_release);
-    }
+    FB_TRY(configure_dp(ctx));
     ctx->dp.last_cells = cells;
-    DpParams P{};
-    P.jobs = jobs;
-    P.meta = d_meta;
+    DpParams P = batch_params(jobs, d_meta, gaps, d_skew, d_path, d_scratch, d_results);
     P.n_jobs = n;
-    P.go = gaps[0]; P.ge = gaps[1]; P.to = gaps[2]; P.te = gaps[3];
-    P.sdirs = d_skew;
-    P.path = d_path;
-    P.scratch = d_scratch;
-    P.results = d_results;
     P.h_results = h_results;
     P.h_path = h_path;
     if (record_events) { FB_CUDA(cudaEventRecord(ctx->ev[0], st)); FB_CUDA(cudaEventRecord(ctx->ev[1], st)); }
-    k_merge_fused<<<grid, kFusedWarps * 32, kFusedWarps * sizeof(WarpShared), st>>>(P, *static_cast<const FusedParams*>(fused_params));
+    k_merge_fused<<<grid, kFusedWarps * 32, kFusedWarps * sizeof(WarpShared), st>>>(P, fused);
     FB_CUDA(cudaGetLastError());
     ctx->launches++;
     if (record_events) { FB_CUDA(cudaEventRecord(ctx->ev[2], st)); FB_CUDA(cudaEventRecord(ctx->ev[3], st)); }
     return FAMSA_OK;
 }
 
-// Bytes of stream-ordered scratch one call of dp_run_device needs at most (it sub-batches above ~1 Gi cells).
+// Runs a batch of merges on the stream: prep, fill, traceback (and the un-skewed direction matrices when d_dirs is set),
+// in sub-batches of consecutive jobs above ~4 Gi cells.
 // jobs[k].p1/p2 hold DEVICE pointers here; widths are the layout widths (upper bounds when ext[k].w*_src is set).
 int dp_run_device(famsa_ctx* ctx, const famsa_dp_job* jobs, const DpJobExt* ext, uint32_t n, const int64_t gaps[4],
                   famsa_dp_result* d_results, uint8_t* d_path, uint8_t* d_dirs, DpMeta** d_meta_out, void** d_blob_out,
-                  cudaStream_t st, const void* fused)
+                  cudaStream_t st)
 {
     DpState& S = ctx->dp;
     std::vector<DpJobDev> dev(n);
     unsigned long long path_off = 0, dirs_off = 0, cells = 0;
     for (uint32_t k = 0; k < n; ++k) {
-        const famsa_dp_job& j = jobs[k];
-        if (j.p1.width == 0 || j.p2.width == 0 || j.p1.card == 0 || j.p2.card == 0) {
-            set_error("dp job " + std::to_string(k) + ": empty profile");
-            return FAMSA_E_INVALID;
-        }
-        if (((unsigned long long)j.p1.width + 1) * (j.p2.width + 1) > 0xffffffffull) {
-            set_error("dp job " + std::to_string(k) + ": more than 2^32 matrix cells");
-            return FAMSA_E_INVALID;
-        }
         DpJobDev& d = dev[k];
-        d.s1 = reinterpret_cast<const long long*>(j.p1.scores); d.c1 = j.p1.counters;
-        d.s2 = reinterpret_cast<const long long*>(j.p2.scores); d.c2 = j.p2.counters;
-        d.w1 = j.p1.width; d.card1 = j.p1.card; d.w2 = j.p2.width; d.card2 = j.p2.card;
-        d.w1_src = ext ? ext[k].w1_src : nullptr; d.w2_src = ext ? ext[k].w2_src : nullptr; d.w_dst = ext ? ext[k].w_dst : nullptr;
+        FB_TRY(make_job(jobs[k], ext ? ext + k : nullptr, k, d));
         d.path_off = path_off; d.dirs_off = dirs_off;           // caller-visible layout: global prefix sums
         path_off += (unsigned long long)d.w1 + d.w2;
         dirs_off += ((unsigned long long)d.w1 + 1) * (d.w2 + 1);
         cells += (unsigned long long)d.w1 * d.w2;
     }
     S.last_cells = cells;
-    // Sub-batches of consecutive jobs bound the device scratch (direction bytes are 1 byte per cell): ~4 Gi cells each.
-    unsigned long long max_cells = 1ull << 32;
-    if (const char* e = getenv("FAMSA_DP_MAX_CELLS")) max_cells = strtoull(e, nullptr, 10);     // development knob
-    uint32_t team_min = kDpTeamMinWidth;
-    if (const char* e = getenv("FAMSA_DP_TEAM_MIN")) team_min = (uint32_t)atoi(e);               // development knob
-    int nw_forced = 0;
-    if (const char* e = getenv("FAMSA_DP_TEAM_WARPS")) nw_forced = atoi(e);                      // development knob
-    uint32_t cluster_min = kDpClusterMinWidth;
-    if (const char* e = getenv("FAMSA_DP_CLUSTER_MIN")) cluster_min = (uint32_t)atoi(e);         // development knob
-    FB_TRY((configure_fill<1, false>(ctx)));
-    FB_TRY((configure_fill<2, false>(ctx)));
-    FB_TRY((configure_fill<4, false>(ctx)));
-    FB_TRY((configure_fill<kDpTeamWarps, false>(ctx)));
-    FB_TRY((configure_fill<4, true>(ctx)));
-    FB_TRY((configure_fill<kDpTeamWarps, true>(ctx)));
-    {
-        static std::atomic<bool> compact_configured[64];
-        if (!compact_configured[ctx->device & 63].load(std::memory_order_acquire)) {
-            FB_CUDA(cudaFuncSetAttribute(k_dp_fill_compact<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * kCompactStride)));
-            FB_CUDA(cudaFuncSetAttribute(k_dp_fill_compact<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(4 * kCompactStride)));
-            FB_CUDA(cudaFuncSetAttribute(k_dp_fill_compact<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(6 * kCompactStride)));
-            compact_configured[ctx->device & 63].store(true, std::memory_order_release);
-        }
-    }
-    {
-        static std::atomic<bool> configured[64];
-        if (!configured[ctx->device & 63].load(std::memory_order_acquire)) {
-            FB_CUDA(cudaFuncSetAttribute(k_merge_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kFusedWarps * sizeof(WarpShared))));
-            configured[ctx->device & 63].store(true, std::memory_order_release);
-        }
-    }
+    const DpKnobs K = read_knobs();
+    FB_TRY(configure_dp(ctx));
 
-    // plan the sub-batches first: one stream-ordered allocation serves all of them
+    // Sub-batches of consecutive jobs bound the device scratch (direction bytes are 1 byte per cell): ~4 Gi cells each.
+    // Plan them first: one stream-ordered allocation serves all of them.
     struct Sub { uint32_t j0, j1; unsigned long long scratch, skew; std::vector<unsigned long long> tblock; };
     std::vector<Sub> subs;
     unsigned long long max_scratch = 64, max_skew = 64;
@@ -1577,7 +1546,7 @@ int dp_run_device(famsa_ctx* ctx, const famsa_dp_job* jobs, const DpJobExt* ext,
         sb.tblock.assign(1, 0);
         while (j1 < n) {
             const unsigned long long mat = ((unsigned long long)dev[j1].w1 + 1) * (dev[j1].w2 + 1);
-            if (j1 > j0 && mat_sum + mat > max_cells) break;
+            if (j1 > j0 && mat_sum + mat > K.max_cells) break;
             dev[j1].scratch_off = scratch_off;
             dev[j1].t_off = t_off;                              // skewed directions are per sub-batch
             scratch_off += Scratch(dev[j1].w1, dev[j1].w2).total;
@@ -1615,26 +1584,12 @@ int dp_run_device(famsa_ctx* ctx, const famsa_dp_job* jobs, const DpJobExt* ext,
     FB_CUDA(cudaEventRecord(ctx->ev[0], st));
     FB_CUDA(cudaEventRecord(ctx->ev[1], st));
     if (n) FB_CUDA(cudaMemcpyAsync(d_jobs, dev.data(), sizeof(DpJobDev) * n, cudaMemcpyHostToDevice, st));
-    if (fused) {
-        if (subs.size() != 1 || d_dirs) { set_error("internal: a fused batch must be one sub-batch without CDPMatrix output"); cudaFreeAsync(blob, st); return FAMSA_E_INVALID; }
-        DpParams P{};
-        P.jobs = d_jobs;
-        P.meta = d_meta;
-        P.order = nullptr;
-        P.n_jobs = n;
-        P.job_base = 0;
-        P.go = gaps[0]; P.ge = gaps[1]; P.to = gaps[2]; P.te = gaps[3];
-        P.dirs = nullptr;
-        P.sdirs = blob + o_skew;
-        P.path = d_path;
-        P.scratch = blob + o_scratch;
-        P.tblock = nullptr;
-        P.results = d_results;
-        k_merge_fused<<<n, kFusedWarps * 32, kFusedWarps * sizeof(WarpShared), st>>>(P, *static_cast<const FusedParams*>(fused));
-        FB_CUDA(cudaGetLastError());
-        ctx->launches++;
-        subs.clear();
-    }
+    DpParams P = batch_params(d_jobs, d_meta, gaps, blob + o_skew, d_path, blob + o_scratch, d_results);
+    P.order = reinterpret_cast<const uint32_t*>(blob + o_order);
+    P.dirs = d_dirs;
+    P.tblock = reinterpret_cast<const unsigned long long*>(blob + o_tblock);
+    const uint32_t sms = (uint32_t)ctx->sm_count;
+    std::vector<int> cls(n);                                     // fill class of each merge: larger = launched first
     for (const Sub& sb : subs) {
         const uint32_t j0 = sb.j0, j1 = sb.j1, m = j1 - j0;
         // rows of the DP matrix as far as the host can tell (the orientation of ProfProf merges is decided on the device)
@@ -1648,160 +1603,118 @@ int dp_run_device(famsa_ctx* ctx, const famsa_dp_job* jobs, const DpJobExt* ext,
         // rest run one warp per merge.  A small batch (the chain-like parts and the top of a guide tree, where a level is
         // one or a few merges) is LATENCY-bound: every merge with more than one stripe gets a cluster of 4-warp blocks,
         // one stripe per SM sub-partition, as many blocks as its stripes can use (up to 16).
-        uint32_t cl_cap = max_cluster4(ctx);
-        if (const char* e = getenv("FAMSA_DP_MAX_CLUSTER")) cl_cap = std::max(1u, std::min(cl_cap, (uint32_t)atoi(e)));   // development knob
+        const uint32_t cl_cap = std::max(1u, std::min(S.cluster4_cap, K.max_cluster));
         // latency mode while the batch's stripes fit one per SM sub-partition
         unsigned long long demand = 0;
         uint32_t n_teamable = 0;
         for (uint32_t a = j0; a < j1; ++a) {
             demand += std::min(stripes_of(a), 4u * cl_cap);
-            n_teamable += std::min(dev[a].w1, dev[a].w2) > team_min;
+            n_teamable += std::min(dev[a].w1, dev[a].w2) > K.team_min;
         }
-        bool small_batch = demand <= 4ull * (unsigned long long)ctx->sm_count;
-        if (const char* e = getenv("FAMSA_DP_LATENCY_MODE")) small_batch = atoi(e) != 0;                 // development knob
+        const bool small_batch = K.latency_mode >= 0 ? K.latency_mode != 0 : demand <= 4ull * sms;
         // throughput mode with only a handful of block-sized merges: give every merge with more than 8 stripes a cluster
-        uint32_t cl_min = cluster_min;
-        if (n_teamable * kDpCluster <= 2u * (uint32_t)ctx->sm_count) cl_min = std::min(cluster_min, std::max(team_min, 256u));
-        const bool duo_on = !getenv("FAMSA_DP_DUO") || atoi(getenv("FAMSA_DP_DUO")) != 0;       // development knob (0: one warp per stripe)
-        const uint32_t duo_cap = duo_on ? max_cluster_duo(ctx) : 1;
-        auto cluster_of = [&](uint32_t a) {                       // latency mode: blocks (of 4 warps) for merge a
-            const uint32_t want = (stripes_of(a) + 3) / 4;
-            uint32_t cl = 1;
-            while (cl < want && cl < cl_cap) cl *= 2;
-            return cl;
-        };
-        auto cls = [&](uint32_t a) -> int {                       // sort key: larger = launched first
+        uint32_t cl_min = K.cluster_min;
+        if (n_teamable * kDpCluster <= 2u * sms) cl_min = std::min(K.cluster_min, std::max(K.team_min, 256u));
+        const uint32_t duo_cap = K.duo ? S.duo_cap : 1;
+        for (uint32_t a = j0; a < j1; ++a) {
             const uint32_t w = std::min(dev[a].w1, dev[a].w2);
             if (small_batch) {
-                if (stripes_of(a) < 2) return 0;
-                const uint32_t cl = cluster_of(a);
+                const uint32_t stripes = stripes_of(a);
+                uint32_t cl = 1;                                 // blocks (of 4 warps) for merge a
+                while (cl < (stripes + 3) / 4 && cl < cl_cap) cl *= 2;
                 // ProfProf merges wide enough for a cluster: producer / consumer pairs (k_dp_fill_duo)
-                if (duo_on && cl >= 2 && dev[a].card1 > 1 && dev[a].card2 > 1) return 100 + (int)std::min(cl, duo_cap);
-                return 10 + (int)cl;
-            }
-            if (w > cl_min) return 2;
-            return w > team_min ? 1 : 0;
-        };
+                if (stripes < 2) cls[a] = 0;
+                else if (K.duo && cl >= 2 && dev[a].card1 > 1 && dev[a].card2 > 1) cls[a] = 100 + (int)std::min(cl, duo_cap);
+                else cls[a] = 10 + (int)cl;
+            } else cls[a] = w > cl_min ? 2 : (w > K.team_min ? 1 : 0);
+        }
         std::vector<uint32_t> order(m);
         std::iota(order.begin(), order.end(), j0);
         std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
-            if (cls(a) != cls(b)) return cls(a) > cls(b);
+            if (cls[a] != cls[b]) return cls[a] > cls[b];
             return (unsigned long long)dev[a].w1 * dev[a].w2 > (unsigned long long)dev[b].w1 * dev[b].w2;
         });
+        // one launch per run [q0, q1) of equal class in `order`
+        std::vector<std::pair<uint32_t, uint32_t>> runs;
+        for (uint32_t q0 = 0, q1 = 0; q0 < m; q0 = q1) {
+            while (q1 < m && cls[order[q1]] == cls[order[q0]]) ++q1;
+            runs.emplace_back(q0, q1);
+        }
 
         // Throughput mode: the first wave of blocks lands on the SMs in launch order, so deal the merges (sorted by size) in
         // snake rows of one block per SM -- the SM that got the largest merge of a row gets the smallest of the next one.
-        if (!small_batch) {
-            const uint32_t sms = (uint32_t)ctx->sm_count;
-            for (uint32_t q0 = 0; q0 < m;) {
-                const int c = cls(order[q0]);
-                uint32_t q1 = q0;
-                while (q1 < m && cls(order[q1]) == c) ++q1;
-                if (c == 1)
+        if (!small_batch)
+            for (const auto& [q0, q1] : runs)
+                if (cls[order[q0]] == 1)
                     for (uint32_t r = q0 + sms, row = 1; r < q1; r += sms, ++row)
                         if (row & 1) std::reverse(order.begin() + r, order.begin() + std::min(q1, r + sms));
-                q0 = q1;
-            }
-        }
 
         // one packed upload: order + tblock
         std::vector<unsigned char> pack(o_scratch - o_order);
         memcpy(pack.data(), order.data(), sizeof(uint32_t) * m);
         memcpy(pack.data() + (o_tblock - o_order), sb.tblock.data(), sizeof(unsigned long long) * (m + 1));
         FB_CUDA(cudaMemcpyAsync(blob + o_order, pack.data(), (o_tblock - o_order) + sizeof(unsigned long long) * (m + 1), cudaMemcpyHostToDevice, st));
-        DpParams P{};
-        P.jobs = d_jobs;
-        P.meta = d_meta;
-        P.order = reinterpret_cast<const uint32_t*>(blob + o_order);
         P.n_jobs = m;
         P.job_base = j0;
-        P.go = gaps[0]; P.ge = gaps[1]; P.to = gaps[2]; P.te = gaps[3];
-        P.dirs = d_dirs;
-        P.sdirs = blob + o_skew;
-        P.path = d_path;
-        P.scratch = blob + o_scratch;
-        P.tblock = reinterpret_cast<const unsigned long long*>(blob + o_tblock);
-        P.results = d_results;
         k_dp_prep<<<m, kPrepThreads, 0, st>>>(P);
         FB_CUDA(cudaGetLastError());
         ctx->launches += 1;
-        // one launch per run of equal class in `order`; different classes run side by side (fork after prep, join before
-        // the traceback) so that a level pays for its slowest merge once, not once per launch shape
-        static const bool debug = getenv("FAMSA_DP_DEBUG") != nullptr;
-        uint32_t n_classes = 0;
-        for (uint32_t q0 = 0; q0 < m;) { const int c = cls(order[q0]); while (q0 < m && cls(order[q0]) == c) ++q0; ++n_classes; }
-        if (n_classes > 1) FB_CUDA(cudaEventRecord(ctx->ev_fork, st));
-        uint32_t class_no = 0, aux_used = 0;
-        cudaStream_t main_st = st;
-        for (uint32_t q0 = 0; q0 < m;) {
-            const int c = cls(order[q0]);
-            uint32_t q1 = q0;
-            while (q1 < m && cls(order[q1]) == c) ++q1;
-            if (debug) fprintf(stderr, "[dp] batch of %u: class %d x %u (first %u x %u, %u stripes), demand %llu, cl_cap %u, latency_mode %d\n", m, c, q1 - q0,
-                               dev[order[q0]].w1, dev[order[q0]].w2, stripes_of(order[q0]), demand, cl_cap, (int)small_batch);
+        // different classes run side by side (fork after prep, join before the traceback) so that a level pays for its
+        // slowest merge once, not once per launch shape
+        if (runs.size() > 1) FB_CUDA(cudaEventRecord(ctx->ev_fork, st));
+        uint32_t aux_used = 0;
+        for (size_t r = 0; r < runs.size(); ++r) {
+            const uint32_t q0 = runs[r].first, q1 = runs[r].second;
+            const int c = cls[order[q0]];
+            if (dp_debug()) fprintf(stderr, "[dp] batch of %u: class %d x %u (first %u x %u, %u stripes), demand %llu, cl_cap %u, latency_mode %d\n", m, c, q1 - q0,
+                                    dev[order[q0]].w1, dev[order[q0]].w2, stripes_of(order[q0]), demand, cl_cap, (int)small_batch);
             DpParams Q = P;
             Q.order = P.order + q0;
             Q.n_jobs = q1 - q0;
             // class 0 (first in launch order is the heaviest) stays on the main stream, the others go to the aux streams
-            cudaStream_t st = main_st;
-            if (class_no > 0) {
-                const uint32_t a = (class_no - 1) % 4;
-                st = ctx->aux_stream[a];
-                if (!(aux_used >> a & 1)) { FB_CUDA(cudaStreamWaitEvent(st, ctx->ev_fork, 0)); aux_used |= 1u << a; }
+            cudaStream_t fst = st;
+            if (r > 0) {
+                const uint32_t a = (uint32_t)(r - 1) % 4;
+                fst = ctx->aux_stream[a];
+                if (!(aux_used >> a & 1)) { FB_CUDA(cudaStreamWaitEvent(fst, ctx->ev_fork, 0)); aux_used |= 1u << a; }
             }
-            ++class_no;
             if (c == 0) {
-                k_dp_fill<1, false><<<(Q.n_jobs + kDpWarps - 1) / kDpWarps, kDpWarps * 32, kDpWarps * sizeof(WarpShared), st>>>(Q);
-                FB_CUDA(cudaGetLastError());
-                ctx->launches++;
+                FB_TRY(launch_fill(ctx, k_dp_fill<1, false>, Q, (Q.n_jobs + kDpWarps - 1) / kDpWarps, kDpWarps * 32, kDpWarps * sizeof(WarpShared), 1, fst));
             } else if (c >= 100) {
-                FB_TRY(launch_duo_fill(ctx, Q, (uint32_t)c - 100, st));
+                const uint32_t cl = (uint32_t)c - 100;
+                FB_TRY(launch_fill(ctx, k_dp_fill_duo, Q, Q.n_jobs * cl, 256, kDuoSmem, cl, fst));
             } else if (c >= 10) {
                 const uint32_t cl = (uint32_t)c - 10;
-                if (cl == 1) {
-                    k_dp_fill<4, false><<<Q.n_jobs, 4 * 32, 4 * sizeof(WarpShared), st>>>(Q);
-                    FB_CUDA(cudaGetLastError());
-                    ctx->launches++;
-                } else FB_TRY(launch_cluster_fill<4>(ctx, Q, cl, st));
+                FB_TRY(launch_fill(ctx, cl == 1 ? k_dp_fill<4, false> : k_dp_fill<4, true>, Q, Q.n_jobs * cl, 4 * 32, 4 * sizeof(WarpShared), cl, fst));
             } else if (c == 2) {
-                FB_TRY(launch_cluster_fill<kDpTeamWarps>(ctx, Q, kDpCluster, st));
+                FB_TRY(launch_fill(ctx, k_dp_fill<kDpTeamWarps, true>, Q, Q.n_jobs * kDpCluster, kDpTeamWarps * 32, kDpTeamWarps * sizeof(WarpShared), kDpCluster, fst));
             } else {
                 // Team size by how many merges there are: every SM holds 8 fill warps (shared memory), so a level with many
                 // block-class merges runs them with smaller teams -- 4 warps from 2 merges per SM on, 2 from 4 -- which lose
                 // less to the ramp-up / ramp-down of the stripe pipeline.
                 // From two merges per SM on, the compact kernel (12 warps per SM): 6, 4 or 2 warps per merge.
                 int nw = kDpTeamWarps;
-                const uint32_t sms = (uint32_t)ctx->sm_count;
-                const int compact_mode = getenv("FAMSA_DP_COMPACT") ? atoi(getenv("FAMSA_DP_COMPACT")) : 1;   // development knob: 0 never, 2 always
-                bool compact = compact_mode == 2 || (compact_mode == 1 && Q.n_jobs >= 2u * sms);
+                bool compact = K.compact == 2 || (K.compact == 1 && Q.n_jobs >= 2u * sms);
                 if (compact) nw = Q.n_jobs >= 6u * sms ? 2 : (Q.n_jobs >= 3u * sms ? 4 : 6);
                 else if (Q.n_jobs >= 4u * sms) nw = 2;
                 else if (Q.n_jobs >= 2u * sms) nw = 4;
-                if (nw_forced) { nw = nw_forced; compact = compact && (nw == 2 || nw == 4 || nw == 6); }
+                if (K.team_warps) { nw = K.team_warps; compact = compact && (nw == 2 || nw == 4 || nw == 6); }
                 if (compact) {
-                    switch (nw) {
-                    case 2: k_dp_fill_compact<2><<<Q.n_jobs, 2 * 32, 2 * kCompactStride, st>>>(Q); break;
-                    case 4: k_dp_fill_compact<4><<<Q.n_jobs, 4 * 32, 4 * kCompactStride, st>>>(Q); break;
-                    default: k_dp_fill_compact<6><<<Q.n_jobs, 6 * 32, 6 * kCompactStride, st>>>(Q); nw = 4; break;
-                    }
-                    FB_CUDA(cudaGetLastError());
-                    ctx->launches++;
+                    const int cw = nw == 2 || nw == 4 ? nw : 6;
+                    FB_TRY(launch_fill(ctx, cw == 2 ? k_dp_fill_compact<2> : (cw == 4 ? k_dp_fill_compact<4> : k_dp_fill_compact<6>), Q, Q.n_jobs, cw * 32,
+                                       cw * kCompactStride, 1, fst));
+                    if (cw == 6) nw = 4;
                     Q.wide_only = 1;                                 // merges whose T needs 8 bytes: the launch below
                 }
-                switch (nw) {
-                case 2: k_dp_fill<2, false><<<Q.n_jobs, 2 * 32, 2 * sizeof(WarpShared), st>>>(Q); break;
-                case 4: k_dp_fill<4, false><<<Q.n_jobs, 4 * 32, 4 * sizeof(WarpShared), st>>>(Q); break;
-                default: k_dp_fill<kDpTeamWarps, false><<<Q.n_jobs, kDpTeamWarps * 32, kDpTeamWarps * sizeof(WarpShared), st>>>(Q); break;
-                }
-                FB_CUDA(cudaGetLastError());
-                ctx->launches++;
+                const int fw = nw == 2 || nw == 4 ? nw : kDpTeamWarps;
+                FB_TRY(launch_fill(ctx, fw == 2 ? k_dp_fill<2, false> : (fw == 4 ? k_dp_fill<4, false> : k_dp_fill<kDpTeamWarps, false>), Q, Q.n_jobs, fw * 32,
+                                   fw * sizeof(WarpShared), 1, fst));
             }
-            q0 = q1;
         }
         for (uint32_t a = 0; a < 4; ++a)
             if (aux_used >> a & 1) {
                 FB_CUDA(cudaEventRecord(ctx->ev_join[a], ctx->aux_stream[a]));
-                FB_CUDA(cudaStreamWaitEvent(main_st, ctx->ev_join[a], 0));
+                FB_CUDA(cudaStreamWaitEvent(st, ctx->ev_join[a], 0));
             }
         k_dp_trace<<<(m + kTraceWarps - 1) / kTraceWarps, kTraceWarps * 32, 0, st>>>(P);
         FB_CUDA(cudaGetLastError());

@@ -22,7 +22,6 @@
 //     those rows -- and rows too long for the register-resident kernel -- are recomputed by
 //     k_lcs_exact, which follows the reference recurrence word for word.
 #include <algorithm>
-#include <atomic>
 #include <cfloat>
 #include <cmath>
 #include <cstring>
@@ -924,20 +923,13 @@ void DevBuf::release()
     cap = 0;
 }
 
-#define FB_TRY(expr)                      \
-    do {                                  \
-        int rc__ = (expr);                \
-        if (rc__ != FAMSA_OK) return rc__; \
-    } while (0)
-
 template <int NL>
 static int launch_tile(famsa_ctx* ctx, const TileParams& P, uint32_t n_tiles, cudaStream_t st)
 {
-    static std::atomic<bool> configured[64];       // per device ordinal; setting the attribute twice is harmless
     const size_t smem = (size_t)blob_words(NL) * 4;
-    if (!configured[ctx->device & 63].load(std::memory_order_acquire)) {
+    if (!(ctx->lcs.tile_configured >> (NL - 1) & 1)) {
         FB_CUDA(cudaFuncSetAttribute(k_lcs_tile<NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured[ctx->device & 63].store(true, std::memory_order_release);
+        ctx->lcs.tile_configured |= 1ull << (NL - 1);
     }
     k_lcs_tile<NL><<<n_tiles, kTileWarps * 32, smem, st>>>(P);
     FB_CUDA(cudaGetLastError());

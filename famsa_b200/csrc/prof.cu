@@ -34,12 +34,6 @@
 
 namespace fb {
 
-#define FB_TRY(expr)                      \
-    do {                                  \
-        int rc__ = (expr);                \
-        if (rc__ != FAMSA_OK) return rc__; \
-    } while (0)
-
 namespace {
 
 __global__ void __launch_bounds__(256) k_prof_leaf(const LeafDesc* __restrict__ leaves, const int8_t* __restrict__ codes,
@@ -187,6 +181,15 @@ void place(ProfState& P, uint32_t id, int slab, size_t* cursor, uint32_t width, 
     ++P.n_live;
 }
 
+// Carves the scratch tables of leaf `ld` (width `width`) out of `base` at *cursor.
+void place_leaf(LeafDesc& ld, unsigned char* base, size_t* cursor, uint32_t width)
+{
+    char* at = reinterpret_cast<char*>(base) + *cursor;
+    ld.scores = reinterpret_cast<long long*>(at);
+    ld.counters = reinterpret_cast<int*>(at + ((size_t)width + 1) * kRows * sizeof(long long));
+    *cursor += table_bytes(width);
+}
+
 int release_entry(famsa_ctx* ctx, uint32_t id)
 {
     ProfState& P = ctx->prof;
@@ -320,6 +323,31 @@ static int prof_resolve(famsa_ctx* ctx, const famsa_prof_merge* merges, uint32_t
     return FAMSA_OK;
 }
 
+// The merged profiles of a batch: one slab, every profile pending and sized for the widest alignment possible (w1 + w2
+// columns); the fill publishes the real width to d_widths[id].  Appends their ids and generations, and one construct job
+// per merge (job index base + k).
+static int new_merged(famsa_ctx* ctx, const std::vector<famsa_dp_job>& jobs, std::vector<DpJobExt>& ext, uint32_t base,
+                      std::vector<uint32_t>& ids, std::vector<uint32_t>& gens, std::vector<ConJobDev>& con)
+{
+    ProfState& P = ctx->prof;
+    size_t slab_bytes = 0;
+    for (const famsa_dp_job& j : jobs) slab_bytes += table_bytes(j.p1.width + j.p2.width);
+    int slab;
+    FB_TRY(new_slab(ctx, slab_bytes, &slab));
+    size_t cur = 0;
+    for (uint32_t k = 0; k < (uint32_t)jobs.size(); ++k) {
+        const uint32_t ub = jobs[k].p1.width + jobs[k].p2.width;
+        const uint32_t id = new_entry(P);
+        place(P, id, slab, &cur, ub, jobs[k].p1.card + jobs[k].p2.card);
+        P.entries[id].pending = true;
+        ids.push_back(id);
+        gens.push_back(P.entries[id].gen);
+        ext[k].w_dst = P.d_widths.as<uint32_t>() + id;
+        con.push_back(ConJobDev{P.entries[id].scores, P.entries[id].counters, base + k, 0});
+    }
+    return FAMSA_OK;
+}
+
 static bool fused_eligible(const std::vector<famsa_dp_job>& jobs)
 {
     if (jobs.size() > 4096) return false;
@@ -370,20 +398,8 @@ static int fused_add(famsa_ctx* ctx, FusedAccum& A, const famsa_prof_merge* merg
 {
     ProfState& P = ctx->prof;
     const uint32_t base = (uint32_t)A.jobs.size();
-    size_t slab_bytes = 0;
-    for (uint32_t k = 0; k < n; ++k) slab_bytes += table_bytes(jobs[k].p1.width + jobs[k].p2.width);
-    int slab;
-    FB_TRY(new_slab(ctx, slab_bytes, &slab));
-    size_t cur = 0;
+    FB_TRY(new_merged(ctx, jobs, ext, base, A.merged_ids, A.merged_gen, A.con));
     for (uint32_t k = 0; k < n; ++k) {
-        const uint32_t ub = jobs[k].p1.width + jobs[k].p2.width;
-        const uint32_t id = new_entry(P);
-        place(P, id, slab, &cur, ub, jobs[k].p1.card + jobs[k].p2.card);
-        P.entries[id].pending = true;
-        A.merged_ids.push_back(id);
-        A.merged_gen.push_back(P.entries[id].gen);
-        ext[k].w_dst = P.d_widths.as<uint32_t>() + id;
-        A.con.push_back(ConJobDev{P.entries[id].scores, P.entries[id].counters, base + k, 0});
         A.dev_bytes_est += fused_dev_estimate(jobs[k]);
         A.path_bytes += align16 ? align_up((uint64_t)jobs[k].p1.width + jobs[k].p2.width, 16) : (uint64_t)jobs[k].p1.width + jobs[k].p2.width;
     }
@@ -434,17 +450,12 @@ static int fused_flush(famsa_ctx* ctx, FusedAccum& A, const int64_t gaps[4], fam
     for (uint32_t k = 0; k < n; ++k) { fj[k].leaf[0].seq = fj[k].leaf[1].seq = 0xffffffffu; fj[k].con = A.con[k]; }
     size_t cur = 0;
     for (size_t a = 0; a < A.leaves.size(); ++a) {
-        const uint32_t k = A.leaf_slot[a].first;
-        const int side = A.leaf_slot[a].second;
-        const uint32_t w = side ? A.jobs[k].p2.width : A.jobs[k].p1.width;
-        char* base = reinterpret_cast<char*>(db + o_leaf + cur);
-        LeafDesc ld = A.leaves[a];
-        ld.scores = reinterpret_cast<long long*>(base);
-        ld.counters = reinterpret_cast<int*>(base + ((size_t)w + 1) * kRows * sizeof(long long));
+        const auto [k, side] = A.leaf_slot[a];
+        LeafDesc& ld = A.leaves[a];
+        place_leaf(ld, db + o_leaf, &cur, side ? A.jobs[k].p2.width : A.jobs[k].p1.width);
         (side ? plan_jobs[k].s2 : plan_jobs[k].s1) = ld.scores;
         (side ? plan_jobs[k].c2 : plan_jobs[k].c1) = ld.counters;
         fj[k].leaf[side] = ld;
-        cur += table_bytes(w);
     }
     memcpy(hj, plan_jobs.data(), sizeof(DpJobDev) * n);
     memcpy(hl, A.level_start.data(), sizeof(uint32_t) * (n_levels + 1));
@@ -455,7 +466,7 @@ static int fused_flush(famsa_ctx* ctx, FusedAccum& A, const int64_t gaps[4], fam
     if (!host_mapped) { FB_CUDA(cudaEventRecord(P.ev[0], st)); FB_CUDA(cudaEventRecord(P.ev[1], st)); }
     const uint32_t grid = std::max(1u, std::min(A.max_level, (uint32_t)ctx->sm_count));      // co-resident: the levels meet at a spin barrier
     FB_TRY(dp_fused_launch(ctx, hj, n, gaps, d_results, db + o_path, reinterpret_cast<DpMeta*>(db + o_meta), db + o_scr, db + o_skew,
-                           host_mapped ? h_results : nullptr, host_mapped ? h_paths : nullptr, &FP, grid, plan.cells, !host_mapped, st));
+                           host_mapped ? h_results : nullptr, host_mapped ? h_paths : nullptr, FP, grid, plan.cells, !host_mapped, st));
     if (!host_mapped) {
         FB_CUDA(cudaEventRecord(P.ev[2], st));
         P.timing_valid = true;
@@ -517,8 +528,7 @@ static int prof_launch(famsa_ctx* ctx, const famsa_prof_merge* merges, uint32_t 
     FB_TRY(ensure_widths(ctx, P.entries.size() + n));
     // A batch of small merges only (the chain-like parts of a guide tree: every level one or a few short merges) runs
     // every merge whole in one block of k_merge_fused instead of five launches.
-    bool fused = fused_eligible(jobs);
-    if (fused) {
+    if (fused_eligible(jobs)) {
         FB_TRY(ensure_rings(ctx));
         FusedAccum A;
         if (fused_fits(ctx, A, jobs)) {
@@ -526,16 +536,19 @@ static int prof_launch(famsa_ctx* ctx, const famsa_prof_merge* merges, uint32_t 
             return fused_flush(ctx, A, gaps, h_results, h_paths, host_mapped, T);
         }
     }
-    // merged tables: one slab per batch, every profile sized for the widest alignment possible (w1 + w2 columns)
-    size_t slab_bytes = 0;
-    for (uint32_t k = 0; k < n; ++k) slab_bytes += table_bytes(jobs[k].p1.width + jobs[k].p2.width);
-    int slab;
-    FB_TRY(new_slab(ctx, slab_bytes, &slab));
-    fused = false;                                                   // (the launch-by-launch path below)
+    T->merged_ids.clear();
+    T->merged_gen.clear();
+    std::vector<ConJobDev> con;
+    FB_TRY(new_merged(ctx, jobs, ext, 0, T->merged_ids, T->merged_gen, con));
+    uint32_t tiles = 0;
+    for (uint32_t k = 0; k < n; ++k) {
+        con[k].tile0 = tiles;
+        tiles += (jobs[k].p1.width + jobs[k].p2.width + 1 + kConTile - 1) / kConTile;
+    }
     // batch blob: [results][con jobs][leaf descs][paths][leaf tables]
     const size_t o_res = 0;
     const size_t o_con = align_up(o_res + sizeof(famsa_dp_result) * n, 256);
-    const size_t o_leafd = align_up(o_con + (fused ? sizeof(FusedJob) : sizeof(ConJobDev)) * n, 256);
+    const size_t o_leafd = align_up(o_con + sizeof(ConJobDev) * n, 256);
     const size_t o_path = align_up(o_leafd + sizeof(LeafDesc) * leaves.size(), 256);
     const size_t o_leaf = align_up(o_path + std::max<uint64_t>(path_need, 1), 256);
     const size_t blob_bytes = o_leaf + leaf_bytes;
@@ -547,47 +560,21 @@ static int prof_launch(famsa_ctx* ctx, const famsa_prof_merge* merges, uint32_t 
     famsa_dp_result* d_results = reinterpret_cast<famsa_dp_result*>(blob + o_res);
     uint8_t* d_path = blob + o_path;
 
+    // one upload: [con jobs][leaf descs]
     std::vector<unsigned char> pack(o_path - o_con);
-    std::vector<ConJobDev> cj_store(n);
-    ConJobDev* cj = cj_store.data();
-    FusedJob* fj = reinterpret_cast<FusedJob*>(pack.data());
+    memcpy(pack.data(), con.data(), sizeof(ConJobDev) * n);
     LeafDesc* ld = reinterpret_cast<LeafDesc*>(pack.data() + (o_leafd - o_con));
-    if (fused)
-        for (uint32_t k = 0; k < n; ++k) fj[k].leaf[0].seq = fj[k].leaf[1].seq = 0xffffffffu;
-    {
-        size_t cur = 0;
-        for (size_t a = 0; a < leaves.size(); ++a) {
-            famsa_dp_profile& p = leaf_slot[a].second ? jobs[leaf_slot[a].first].p2 : jobs[leaf_slot[a].first].p1;
-            char* base = reinterpret_cast<char*>(blob + o_leaf + cur);
-            leaves[a].scores = reinterpret_cast<long long*>(base);
-            leaves[a].counters = reinterpret_cast<int*>(base + ((size_t)p.width + 1) * kRows * sizeof(long long));
-            p.scores = reinterpret_cast<const int64_t*>(leaves[a].scores);
-            p.counters = leaves[a].counters;
-            cur += table_bytes(p.width);
-            ld[a] = leaves[a];
-            if (fused) fj[leaf_slot[a].first].leaf[leaf_slot[a].second] = leaves[a];
-        }
-    }
-    T->merged_ids.assign(n, 0);
-    T->merged_gen.assign(n, 0);
     size_t cur = 0;
-    uint32_t tiles = 0;
-    for (uint32_t k = 0; k < n; ++k) {
-        const uint32_t ub = jobs[k].p1.width + jobs[k].p2.width;
-        const uint32_t id = new_entry(P);
-        place(P, id, slab, &cur, ub, jobs[k].p1.card + jobs[k].p2.card);
-        P.entries[id].pending = true;
-        T->merged_ids[k] = id;
-        T->merged_gen[k] = P.entries[id].gen;
-        ext[k].w_dst = P.d_widths.as<uint32_t>() + id;
-        cj[k].os = P.entries[id].scores; cj[k].oc = P.entries[id].counters; cj[k].job = k; cj[k].tile0 = tiles;
-        tiles += (ub + 1 + kConTile - 1) / kConTile;
-        if (fused) fj[k].con = cj[k];
+    for (size_t a = 0; a < leaves.size(); ++a) {
+        famsa_dp_profile& p = leaf_slot[a].second ? jobs[leaf_slot[a].first].p2 : jobs[leaf_slot[a].first].p1;
+        place_leaf(leaves[a], blob + o_leaf, &cur, p.width);
+        p.scores = reinterpret_cast<const int64_t*>(leaves[a].scores);
+        p.counters = leaves[a].counters;
+        ld[a] = leaves[a];
     }
-    if (!fused) memcpy(pack.data(), cj, sizeof(ConJobDev) * n);
     FB_CUDA(cudaEventRecord(P.ev[0], st));
     FB_CUDA(cudaMemcpyAsync(blob + o_con, pack.data(), pack.size(), cudaMemcpyHostToDevice, st));
-    if (!leaves.empty() && !fused) {
+    if (!leaves.empty()) {
         k_prof_leaf<<<(unsigned)leaves.size(), 256, 0, st>>>(reinterpret_cast<const LeafDesc*>(blob + o_leafd), L.d_raw_codes.as<int8_t>(),
                                                              L.d_raw_off.as<uint64_t>(), L.d_raw_len.as<uint32_t>(),
                                                              P.d_sm.as<long long>(), gaps[0], gaps[1], gaps[2], gaps[3]);
@@ -599,12 +586,10 @@ static int prof_launch(famsa_ctx* ctx, const famsa_prof_merge* merges, uint32_t 
     void* dp_blob = nullptr;
     FB_TRY(dp_run_device(ctx, jobs.data(), ext.data(), n, gaps, d_results, d_path, nullptr, &d_meta, &dp_blob, st));
     FB_CUDA(cudaEventRecord(P.ev[1], st));
-    if (!fused) {
-        k_prof_construct<<<tiles, kConThreads, 0, st>>>(reinterpret_cast<const ConJobDev*>(blob + o_con), n, d_meta, d_results, d_path,
-                                                        gaps[0], gaps[1], gaps[2], gaps[3]);
-        FB_CUDA(cudaGetLastError());
-        ++ctx->launches;
-    }
+    k_prof_construct<<<tiles, kConThreads, 0, st>>>(reinterpret_cast<const ConJobDev*>(blob + o_con), n, d_meta, d_results, d_path,
+                                                    gaps[0], gaps[1], gaps[2], gaps[3]);
+    FB_CUDA(cudaGetLastError());
+    ++ctx->launches;
     FB_CUDA(cudaEventRecord(P.ev[2], st));
     P.timing_valid = true;
     FB_CUDA(cudaMemcpyAsync(h_results, d_results, sizeof(famsa_dp_result) * n, cudaMemcpyDeviceToHost, st));
@@ -785,7 +770,7 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
         f.merge_ids = acc_merges;
         f.path_base = acc_path_base;
         f.res_base = acc_res_base;
-        if (getenv("FAMSA_DP_DEBUG")) fprintf(stderr, "[tree] fused launch: %u levels, %zu merges\n", acc_levels, acc.jobs.size());
+        if (dp_debug()) fprintf(stderr, "[tree] fused launch: %u levels, %zu merges\n", acc_levels, acc.jobs.size());
         const auto t0 = now();
         const int r = fused_flush(ctx, acc, gaps, P.h_tree_results + acc_res_base, P.h_tree_paths + acc_path_base, true, &f.t);
         t_launch += std::chrono::duration<double, std::micro>(now() - t0).count();
@@ -796,11 +781,17 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
         max_in_flight = std::max<uint32_t>(max_in_flight, (uint32_t)q.size());
         return FAMSA_OK;
     };
+    auto finished = [&](const ProfTicket& t) { return t.done_seq ? *P.h_done >= t.done_seq : (!t.done || cudaEventQuery(t.done) == cudaSuccess); };
     for (size_t lv = 0; lv < levels.size() && rc == FAMSA_OK; ++lv) {
         const std::vector<uint32_t>& level = levels[lv];
+        std::vector<famsa_prof_merge> mg(level.size());
+        for (size_t a = 0; a < level.size(); ++a) {
+            const uint32_t k = level[a];
+            mg[a].child1 = handle[(uint32_t)tree[2 * k]];
+            mg[a].child2 = handle[(uint32_t)tree[2 * k + 1]];
+        }
         {
             // small merges: join the accumulation when the level fits
-            auto finished = [&](const ProfTicket& t) { return t.done_seq ? *P.h_done >= t.done_seq : (!t.done || cudaEventQuery(t.done) == cudaSuccess); };
             while (!q.empty() && finished(q.front().t) && rc == FAMSA_OK) rc = collect_front();
             if (rc) break;
             // A queued child is known by an upper bound only (the sum of its children's bounds), and along a chain the bounds
@@ -817,12 +808,6 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
                 while (!q.empty() && rc == FAMSA_OK) rc = collect_front();
                 if (rc) break;
                 ++n_drains;
-            }
-            std::vector<famsa_prof_merge> mg(level.size());
-            for (size_t a = 0; a < level.size(); ++a) {
-                const uint32_t k = level[a];
-                mg[a].child1 = handle[(uint32_t)tree[2 * k]];
-                mg[a].child2 = handle[(uint32_t)tree[2 * k + 1]];
             }
             std::vector<famsa_dp_job> jobs;
             std::vector<DpJobExt> ext;
@@ -860,12 +845,11 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
                     continue;
                 }
             }
-            if (getenv("FAMSA_DP_DEBUG")) fprintf(stderr, "[tree] level %zu (%zu merges) not fused: eligible %d, path room %d\n", lv, level.size(), (int)fused_eligible(jobs), (int)(path_cursor + path_need <= P.h_tree_paths_cap)), fprintf(stderr, "        first job: %u (card %u) x %u (card %u)\n", jobs[0].p1.width, jobs[0].p1.card, jobs[0].p2.width, jobs[0].p2.card);
+            if (dp_debug()) fprintf(stderr, "[tree] level %zu (%zu merges) not fused: eligible %d, path room %d\n", lv, level.size(), (int)fused_eligible(jobs), (int)(path_cursor + path_need <= P.h_tree_paths_cap)), fprintf(stderr, "        first job: %u (card %u) x %u (card %u)\n", jobs[0].p1.width, jobs[0].p1.card, jobs[0].p2.width, jobs[0].p2.card);
             rc = flush_acc();                                         // this level goes launch by launch: everything before it first
             if (rc) break;
         }
         // collect whatever has finished already (tightens the bounds for free)
-        auto finished = [&](const ProfTicket& t) { return t.done_seq ? *P.h_done >= t.done_seq : (!t.done || cudaEventQuery(t.done) == cudaSuccess); };
         while (!q.empty() && finished(q.front().t) && rc == FAMSA_OK) rc = collect_front();
         if (rc) break;
         auto level_cost = [&](uint64_t* bound_cells, uint64_t* path_need) {
@@ -901,12 +885,6 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
                 cudaFreeHost(old);
             }
         }
-        std::vector<famsa_prof_merge> mg(level.size());
-        for (size_t a = 0; a < level.size(); ++a) {
-            const uint32_t k = level[a];
-            mg[a].child1 = handle[(uint32_t)tree[2 * k]];
-            mg[a].child2 = handle[(uint32_t)tree[2 * k + 1]];
-        }
         q.emplace_back();
         InFlight& f = q.back();
         f.merge_ids = level;
@@ -931,7 +909,7 @@ int prof_align_tree(famsa_ctx* ctx, const int32_t* tree, uint32_t n_leaves, cons
     if (rc == FAMSA_OK) rc = flush_acc();
     while (!q.empty()) { const int r2 = collect_front(); if (rc == FAMSA_OK) rc = r2; }
     if (rc) return rc;
-    if (getenv("FAMSA_DP_DEBUG"))
+    if (dp_debug())
         fprintf(stderr, "[tree] host time: %.0f us in prof_launch, %.0f us waiting in prof_collect, %.0f us total so far, %u batches\n", t_launch, t_collect,
                 std::chrono::duration<double, std::micro>(now() - t_begin).count(), n_batches);
     FB_CUDA(cudaEventRecord(P.ev_tree[1], ctx->stream));
